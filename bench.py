@@ -3,6 +3,7 @@
 
     python bench.py --gpus N --steps K --warmup W [--config NAME]   # this repo's CUDA path
     python bench.py --impl reference --gpus N --steps K ...         # the CPU oracle (reference arm)
+    python bench.py ... --dump-outputs DIR                          # also write the last timed step's outputs as .npy
 
 Configs (BASELINE.json `configs`):
     query_vith   (default) configs[2] / [3]: RSPrompter-query ViT-H bf16, bs 8 per GPU, 1024^2, 100 queries
@@ -233,7 +234,7 @@ def run_reference(args) -> None:
     run = _oracle_setup(args)
     size = args.size if CONFIGS[args.config]["variant"] == "encoder" else SIZE
     xs = [_oracle_preprocess(_u8_images(1, size, s)) for s in range(2)]
-    budget = 240.0
+    budget = 60.0      # seconds of warmup at most
     t_start = time.perf_counter()
     w_done = 0
     times = []
@@ -241,14 +242,12 @@ def run_reference(args) -> None:
         for i in range(args.warmup):
             run(xs[i % 2])
             w_done += 1
-            if time.perf_counter() - t_start > budget * 0.25:
+            if time.perf_counter() - t_start > budget:
                 break
-        for i in range(max(args.steps, 5)):
+        for i in range(args.steps):
             t0 = time.perf_counter()
             run(xs[i % 2])
             times.append(time.perf_counter() - t0)
-            if time.perf_counter() - t_start > budget and len(times) >= 2:
-                break
     total = sum(times)
     val = len(times) / total
     line = dict(metric="images/sec", value=val, unit="images/s", n_gpus=args.gpus, steps=len(times),
@@ -356,6 +355,43 @@ def _roofline(model_step, trace_fn, inst_steps: int, step_ms: float, peaks: dict
             out["traffic"] = sum(k["dram_read_bytes"] + k["dram_write_bytes"] for k in g) / sum(k["launches"] for k in g)
             out["traffic_source"] = f"profiles/r02_traffic_{args.config}.json (ncu capture of one step, mean bytes per GEMM launch)"
     return out
+
+
+DUMP_BYTES = 64 << 20      # --dump-outputs writes at most this much
+MASK_SAMPLE = 4096         # mask pixels per instance slot written by --dump-outputs (the same seeded positions for all)
+
+
+def dump_outputs(out_dir: str, host_buf: torch.Tensor, rec0, variant: str, size: int) -> None:
+    """Write what one end-to-end step handed its caller in host memory (rank 0's batch) as DIR/<name>.npy.
+
+    encoder:   image_embeddings  f32 [B, 256, S/16, S/16] (a flat seeded sample if larger than DUMP_BYTES)
+    detectors: counts f64 [B]; rows f32 [B, M, 6] (x1, y1, x2, y2, score, label); mask_area f64 [B, M] (set pixels of
+               each mask); mask_sample f32 [B, M, MASK_SAMPLE] (each mask at MASK_SAMPLE pixels drawn with seed 0).
+               Slots at or beyond an image's count are written as zeros."""
+    import numpy as np
+    g = torch.Generator().manual_seed(0)
+    if variant == "encoder":
+        emb = host_buf.view(torch.float32).view(BATCH, 256, size // 16, size // 16)
+        if emb.numel() * 4 > DUMP_BYTES:
+            idx = torch.randperm(emb.numel(), generator=g)[:DUMP_BYTES // 4].sort().values
+            arrays = dict(image_embeddings_sample=emb.reshape(-1)[idx])
+        else:
+            arrays = dict(image_embeddings=emb)
+    else:
+        rec = rec0.like(host_buf)
+        H, W = rec.hw
+        valid = torch.arange(rec.slots)[None, :] < rec.counts[:, None].long()
+        bits = rec.mask_bits.reshape(rec.batch, rec.slots, H * W // 8)
+        pix = torch.randperm(H * W, generator=g)[:MASK_SAMPLE]
+        sample = (bits[..., pix // 8] >> (pix % 8).to(torch.uint8)) & 1
+        area = sum(((bits >> k) & 1).sum(-1, dtype=torch.int64) for k in range(8))
+        v = valid[..., None]
+        arrays = dict(counts=rec.counts.double(), rows=torch.where(v, rec.rows, 0.0),
+                      mask_area=torch.where(valid, area.double(), 0.0), mask_sample=torch.where(v, sample.float(), 0.0))
+    assert sum(a.numel() * a.element_size() for a in arrays.values()) <= DUMP_BYTES
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, f"{name}.npy"), a.contiguous().numpy())
 
 
 def run_ours(args) -> None:
@@ -523,6 +559,9 @@ def run_ours(args) -> None:
         ms = timed(step_resident, args.steps)
         launches = _lib.launch_count - l0
         ms_e2e = timed(step_e2e, args.steps)
+    if args.dump_outputs and rank == 0:     # the host buffer the last timed step's record / embedding was copied to
+        dump_outputs(args.dump_outputs, hbuf[(args.steps - 1) % 2], None if variant == "encoder" else rec0,
+                     variant, size)
 
     peaks = _peaks()
     roof, roof_err = None, None
@@ -590,7 +629,15 @@ def main():
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--config", default="query_vith", choices=sorted(CONFIGS))
     ap.add_argument("--size", type=int, default=1024, help="image size of the encoder_vith config (512/768/1024/1280)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last end-to-end step returned (rank 0's batch) as "
+                         "DIR/<name>.npy, float32 / float64, at most 64 MB; the inputs are seeded, so runs with the "
+                         "same arguments can be compared output for output")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the outputs of --impl ours")
     if args.impl == "reference":
         run_reference(args)
     else:

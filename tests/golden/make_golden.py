@@ -382,11 +382,41 @@ def main_necks():
     print("wrote", path, os.path.getsize(path), {k: list(v.keys()) for k, v in fx.items()})
 
 
+CONFIG_NAMES = ("rsprompter_anchor-nwpu.py", "rsprompter_anchor-nwpu-peft-512.py", "rsprompter_query-nwpu.py",
+                "rsprompter_query-nwpu-peft-512.py", "samdet-nwpu.py", "samseg-maskrcnn-nwpu.py",
+                "samseg-mask2former-nwpu.py")
+
+
+def main_configs():
+    """tests/golden/reference_configs.pt: the reference's own configs/rsprompter/*-nwpu*.py resolved through their
+    ``_base_`` chains by rsprompter_b200.registry.Config (mmengine's merge rules), per file the ``model`` dict and
+    ``custom_imports`` as plain dicts (tuples and ranges kept).  Needs the built package."""
+    sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.dirname(os.path.abspath(__file__)))))
+    from rsprompter_b200.registry import Config
+
+    def plain(o):
+        if isinstance(o, dict):
+            return {k: plain(v) for k, v in o.items()}
+        if isinstance(o, (list, tuple)):
+            return type(o)(plain(v) for v in o)
+        return o
+
+    fx = {}
+    for name in CONFIG_NAMES:
+        cfg = Config.fromfile(os.path.join(REF, "configs", "rsprompter", name)).to_dict()
+        fx[name] = dict(model=plain(cfg["model"]), custom_imports=plain(cfg["custom_imports"]))
+    path = os.path.join(os.path.dirname(OUT), "reference_configs.pt")
+    torch.save(fx, path)
+    print("wrote", path, os.path.getsize(path), sorted(fx))
+
+
 if __name__ == "__main__":
     if not os.path.isdir(REF):
         sys.exit("/root/reference not mounted")
     if "maskrcnn" in sys.argv[1:]:
         main_maskrcnn()
+    elif "configs" in sys.argv[1:]:
+        main_configs()
     elif "state_keys" in sys.argv[1:]:
         main_state_keys()
     elif "necks" in sys.argv[1:]:

@@ -1,12 +1,19 @@
-"""The reference's own config files load unchanged through the registry surface and build the B200
-modules (skipped where /root/reference is not mounted, e.g. on the GPU box)."""
+"""The reference's own config files (configs/rsprompter/*-nwpu*.py) build the B200 modules through the registry
+surface.  tests/golden/reference_configs.pt holds each file resolved through its ``_base_`` chain (``model`` and
+``custom_imports``; tests/golden/make_golden.py configs)."""
+import copy
 import os
 
 import pytest
 import torch
 
-REF_CFG = "/root/reference/configs/rsprompter"
-pytestmark = pytest.mark.skipif(not os.path.isdir(REF_CFG), reason="reference tree not mounted")
+FX = torch.load(os.path.join(os.path.dirname(__file__), "golden", "reference_configs.pt"), weights_only=False)
+
+
+def _load(name):
+    """The resolved reference config file `name` as a Config."""
+    from rsprompter_b200.registry import Config
+    return Config(copy.deepcopy(FX[name]), filename=name)
 
 
 def _strip_init(cfg):
@@ -21,9 +28,20 @@ def _strip_init(cfg):
     return cfg
 
 
-def test_base_config_inheritance_and_delete():
+def test_base_config_inheritance_and_delete(tmp_path):
+    """Config.fromfile merges a child over its ``_base_`` the way rsprompter_anchor-nwpu-peft-512.py sits on
+    _base_/rsprompter_anchor.py: ``backbone`` and ``neck.feature_aggregator`` are replaced (``_delete_=True``), the rest
+    of the model, ``neck.feature_spliter`` included, is inherited."""
     from rsprompter_b200.registry import Config
-    cfg = Config.fromfile(os.path.join(REF_CFG, "rsprompter_anchor-nwpu-peft-512.py"))
+    base, peft = FX["rsprompter_anchor-nwpu.py"], FX["rsprompter_anchor-nwpu-peft-512.py"]
+    assert "extra_config" in base["model"]["backbone"]
+    (tmp_path / "_base_").mkdir()
+    (tmp_path / "_base_" / "base.py").write_text(
+        f"custom_imports = {base['custom_imports']!r}\nmodel = {base['model']!r}\n")
+    child = dict(backbone=dict(_delete_=True, **peft["model"]["backbone"]),
+                 neck=dict(feature_aggregator=dict(_delete_=True, **peft["model"]["neck"]["feature_aggregator"])))
+    (tmp_path / "child.py").write_text(f"_base_ = ['_base_/base.py']\nmodel = {child!r}\n")
+    cfg = Config.fromfile(str(tmp_path / "child.py"))
     m = cfg.model
     assert m.type == "RSPrompterAnchor"                                   # from _base_
     assert m.backbone.type == "MMPretrainSamVisionEncoder" and "extra_config" not in m.backbone  # _delete_
@@ -32,14 +50,16 @@ def test_base_config_inheritance_and_delete():
     assert m.roi_head.bbox_head.num_classes == 10
     assert m.test_cfg.rcnn.max_per_img == 100
     assert cfg.custom_imports["imports"] == ["mmdet.rsprompter"]
+    ref = _load("rsprompter_anchor-nwpu-peft-512.py").model
+    assert m.backbone == ref.backbone and m.neck == ref.neck
 
 
 @pytest.mark.parametrize("name,enc_cls", [("rsprompter_anchor-nwpu.py", "RSSamVisionEncoder"),
                                           ("rsprompter_anchor-nwpu-peft-512.py", "MMPretrainSamVisionEncoder")])
 def test_reference_anchor_configs_build(name, enc_cls):
     from rsprompter_b200 import synthetic
-    from rsprompter_b200.registry import MODELS, Config
-    cfg = Config.fromfile(os.path.join(REF_CFG, name))
+    from rsprompter_b200.registry import MODELS
+    cfg = _load(name)
     model_cfg = _strip_init(cfg.to_dict()["model"])
     model = MODELS.build(model_cfg)
     assert type(model).__name__ == "RSPrompterAnchor"
@@ -61,8 +81,8 @@ def test_reference_anchor_configs_build(name, enc_cls):
                                              ("rsprompter_query-nwpu-peft-512.py", "MMPretrainSamVisionEncoder", 70)])
 def test_reference_query_configs_build(name, enc_cls, nq):
     from rsprompter_b200 import synthetic
-    from rsprompter_b200.registry import MODELS, Config
-    cfg = Config.fromfile(os.path.join(REF_CFG, name))
+    from rsprompter_b200.registry import MODELS
+    cfg = _load(name)
     model_cfg = _strip_init(cfg.to_dict()["model"])
     model = MODELS.build(model_cfg)
     assert type(model).__name__ == "RSPrompterQuery" and type(model.backbone).__name__ == enc_cls
@@ -81,8 +101,8 @@ def test_reference_samdet_config_builds_the_segmentor():
     """configs/rsprompter/samdet-nwpu.py: type SAMDet with a stock mmdet FasterRCNN detector (outside this package) and
     an RSSamModel segmentor (SURVEY 8(f4), M:718-741, 1060-1215): the segmentor entry builds the B200 SamModel
     (ViT-B: samdet-nwpu.py:25 points at sam_vit_base) with HF SamModel's parameter names; SAMDet is in the registry."""
-    from rsprompter_b200.registry import MODELS, Config
-    cfg = Config.fromfile(os.path.join(REF_CFG, "samdet-nwpu.py"))
+    from rsprompter_b200.registry import MODELS
+    cfg = _load("samdet-nwpu.py")
     m = cfg.to_dict()["model"]
     assert m["type"] == "SAMDet" and MODELS.get("SAMDet") is not None
     assert m["segmentor"]["type"] == "RSSamModel" and m["detector"]["type"] == "FasterRCNN"
@@ -102,8 +122,8 @@ def test_reference_samseg_maskrcnn_config_builds():
     StandardRoIHead / Shared2FCBBoxHead / FCNMaskHead builds from the reference's own config file and takes a state dict
     with mmdet's parameter names (fcn_mask_head.py:68-126: convs.N.conv, upsample, conv_logits)."""
     from rsprompter_b200 import synthetic
-    from rsprompter_b200.registry import MODELS, Config
-    cfg = Config.fromfile(os.path.join(REF_CFG, "samseg-maskrcnn-nwpu.py"))
+    from rsprompter_b200.registry import MODELS
+    cfg = _load("samseg-maskrcnn-nwpu.py")
     model = MODELS.build(_strip_init(cfg.to_dict()["model"]))
     assert type(model).__name__ == "SAMSegMaskRCNN" and type(model.roi_head).__name__ == "StandardRoIHead"
     assert type(model.roi_head.mask_head).__name__ == "FCNMaskHead" and model.roi_head.mask_head.num_classes == 10
@@ -123,8 +143,8 @@ def test_reference_samseg_mask2former_config_builds():
     Mask2FormerHead (feat_channels 256, 9 decoder layers, FFN 2048) / MaskFormerFusionHead builds from the reference's
     own config file and takes a state dict with mmdet's parameter names."""
     from rsprompter_b200 import synthetic
-    from rsprompter_b200.registry import MODELS, Config
-    cfg = Config.fromfile(os.path.join(REF_CFG, "samseg-mask2former-nwpu.py"))
+    from rsprompter_b200.registry import MODELS
+    cfg = _load("samseg-mask2former-nwpu.py")
     model = MODELS.build(_strip_init(cfg.to_dict()["model"]))
     assert type(model).__name__ == "SAMSegMask2Former" and type(model.panoptic_head).__name__ == "Mask2FormerHead"
     assert type(model.panoptic_fusion_head).__name__ == "MaskFormerFusionHead"
